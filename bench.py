@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - WHENet per-crop forward throughput on B200 (see the contract in the task + DESIGN.md).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--precision bf16] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--precision bf16] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (reference whenet.py:22-34) over one batch of B synthetic
 224x224x3 uint8 crops per GPU (default B=512: BASELINE.json configs[2]; at N GPUs the global batch
@@ -136,8 +136,11 @@ def run_reference(args):
         port.get_angle(crops)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        port.get_angle(crops)
+        out = port.get_angle(crops)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "angles.npy"), np.stack(out, axis=1).astype(np.float32))
     v = sample * args.steps / dt
     line = {"impl": "reference", "metric": METRIC, "value": v, "unit": "crops/s", "n_gpus": args.gpus,
             "steps": args.steps, "warmup": args.warmup, "ms_per_step": dt / args.steps * 1e3, "higher_is_better": True,
@@ -162,6 +165,9 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--chunk", type=int, default=0)
     ap.add_argument("--opt", action="append", default=[], help="library option key=value (repeatable)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the angles of the last timed step to DIR/angles.npy (float32, [N*B, 3] yaw/pitch/roll in "
+                         "degrees); the seeded inputs make two builds comparable output for output")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -244,6 +250,9 @@ def main():
     ms = e0.elapsed_time(e1)
     launches = net.launch_count() - l0
     clocks = sampler.finish() if sampler else None
+    if args.dump_outputs and rank == 0:      # before the e2e and profile legs below reuse `angles`
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "angles.npy"), (gathered if world > 1 else angles).cpu().numpy())
     t = torch.tensor([ms], device="cuda")
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

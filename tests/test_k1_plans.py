@@ -6,22 +6,21 @@ import subprocess
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-EXE = os.path.join(ROOT, "build_tmp", "k1_plan_dump")
 LINE = re.compile(r"b(\d+)\s+(\d+)->\s*(\d+) k(\d) s(\d) cin\s*(\d+) cexp\s*(\d+) :\s*(\d+)x(\d+)\s+r(\d) cc(\d+)\s+nt(\d+) nb(\d)\s+mtiles (\d) "
                   r"rows_alloc\s+(\d+) tmem\s+(\d+) chunks\s+(\d+) PY\s+(\d+) PYc\s+(\d+) smem\s+(\d+) \(A\s+(\d+) W\s+(\d+) C\s+(\d+) E\s+(\d+)\) (\d)/SM")
 KEYS = "idx hin ho k s cin cexp th tw r cc nt nb mtiles rows_alloc tmem chunks PY PYc smem A W C E per_sm".split()
 
 
 @pytest.fixture(scope="module")
-def dump():
-    os.makedirs(os.path.dirname(EXE), exist_ok=True)
+def dump(tmp_path_factory):
+    exe = str(tmp_path_factory.mktemp("plans") / "k1_plan_dump")
     nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-    r = subprocess.run([nvcc, "-std=c++17", "-arch=sm_100a", "-o", EXE, os.path.join(ROOT, "tools", "k1_plan_dump.cu")],
+    r = subprocess.run([nvcc, "-std=c++17", "-arch=sm_100a", "-o", exe, os.path.join(ROOT, "tools", "k1_plan_dump.cu")],
                        capture_output=True, text=True)
     assert r.returncode == 0, r.stderr
 
     def run(*plan):
-        out = subprocess.run([EXE] + [str(v) for v in plan], capture_output=True, text=True, check=True).stdout
+        out = subprocess.run([exe] + [str(v) for v in plan], capture_output=True, text=True, check=True).stdout
         rows = []
         for line in out.splitlines():
             m = LINE.search(line)

@@ -8,20 +8,19 @@ import subprocess
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-EXE = os.path.join(ROOT, "build_tmp", "route_plan_dump")
 SMEM_OPTIN = 227 * 1024          # dynamic + static shared memory one CTA may use on sm_100
 
 
 @pytest.fixture(scope="module")
-def dump():
-    os.makedirs(os.path.dirname(EXE), exist_ok=True)
+def dump(tmp_path_factory):
+    exe = str(tmp_path_factory.mktemp("plans") / "route_plan_dump")
     nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-    r = subprocess.run([nvcc, "-std=c++17", "-arch=sm_100a", "-o", EXE, os.path.join(ROOT, "tools", "route_plan_dump.cu")],
+    r = subprocess.run([nvcc, "-std=c++17", "-arch=sm_100a", "-o", exe, os.path.join(ROOT, "tools", "route_plan_dump.cu")],
                        capture_output=True, text=True)
     assert r.returncode == 0, r.stderr
 
     def run(crops):
-        out = subprocess.run([EXE, str(crops)], capture_output=True, text=True, check=True).stdout
+        out = subprocess.run([exe, str(crops)], capture_output=True, text=True, check=True).stdout
         kd, k2, pw3 = {}, {}, {}
         for line in out.splitlines():
             m = re.search(r"kd b(\d+) cc (\d+) threads (\d+) strips (\d+) pw (\d+) smem (\d+) chunks (\d+)", line)
